@@ -16,6 +16,8 @@ GEMM+leapfrog passes, MH test + select, dual-averaging update.
                                              the north_star's 8-GPU point
     python bench.py --workload iwae ...      the other half of BASELINE.json's metric:
                                              particle-ELBOs/s, VAE IWAE K=64, batch 4096/GPU
+    python bench.py --dump-outputs DIR ...   also write the last timed step's outputs as
+                                             DIR/<name>.npy, to compare two builds
 
 Chains shard across ranks with no data-path collective; the only exchange is
 ONE packed all-reduce per iteration: [sum acc, n] + the EWMV statistics
@@ -99,7 +101,34 @@ def parse():
     ap.add_argument("--no-adapt", action="store_true",
                     help="kernel-timing experiments only: fixed step size, no "
                          "adaptation (not the benchmark configuration)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as "
+                         "DIR/<name>.npy (rank 0; see dump_outputs)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
+
+
+DUMP_ROWS = 4096
+
+
+def dump_outputs(path, arrays):
+    """Write {name: tensor} as path/<name>.npy in float32 (float64 stays float64).  Arrays with
+    more than DUMP_ROWS rows keep the same seeded sample of DUMP_ROWS rows (one per chain or
+    datum, aligned across the arrays), so the files stay below 64 MB and two builds run with
+    the same arguments can be compared file by file."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.dim() > 0 and t.shape[0] > DUMP_ROWS:
+            rows = np.sort(np.random.Generator(np.random.PCG64(0)).choice(
+                t.shape[0], DUMP_ROWS, replace=False))
+            t = t[torch.as_tensor(rows, device=t.device)]
+        if t.dtype != torch.float64:
+            t = t.float()
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
 
 
 def load_peaks():
@@ -379,6 +408,9 @@ def run_iwae(args):
         td.barrier()
     if sampler:
         sampler.mark_end("timed")
+    if args.dump_outputs and rank == 0:     # before the e2e steps overwrite them
+        dump_outputs(args.dump_outputs,
+                     dict(cost=cost, **{"grad_" + k: v for k, v in zip(W, g)}))
     launches = lib.launches - launches0
     if launches_per_replay is not None:
         launches = launches_per_replay * args.steps
@@ -547,6 +579,13 @@ def run_hmc(args):
     value = C * world * L * args.steps / (total_ms * 1e-3)
     acc_mean = float(info.acceptance_rate.mean())
     step_size = float(info.updated_step_size)
+    if args.dump_outputs and rank == 0:     # before the e2e steps overwrite them
+        dump_outputs(args.dump_outputs, {
+            "samples_x": info.samples["x"], "init_momentum_x": info.init_momentum["x"],
+            "acceptance_rate": info.acceptance_rate,
+            "updated_step_size": info.updated_step_size,
+            "orig_hamiltonian": info.orig_hamiltonian, "hamiltonian": info.hamiltonian,
+            "orig_log_prob": info.orig_log_prob, "log_prob": info.log_prob})
 
     # ---------------- e2e: host buffers through the public API ---------------
     # Every step: H2D of the step's chain state from pinned host memory, one

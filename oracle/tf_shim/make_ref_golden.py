@@ -8,7 +8,9 @@ of the reference (tf.random_normal hmc.py:22 / sgmcmc.py:196-365, tf.random_unif
 replaced by injected arrays, which are stored next to the outputs; the per-iteration booleans are
 fed through placeholders exactly as the reference's examples do (hmc.py:228-231).
 """
+import hashlib
 import importlib
+import json
 import os
 import sys
 import types
@@ -535,6 +537,19 @@ def run_reference_hmc_big(name):
     return {k: np.stack(v) for k, v in rec.items()}
 
 
+# per-iteration outputs of run_reference_hmc_big kept in tests/golden/ref_<name>_l50.npz (the
+# chain states are left out: [iters, C, D] would not fit a fixture at D = 1024)
+BIG_KEYS = ("acc", "step_size", "lp0", "h0", "h1")
+
+
+def write_reference_hmc_big():
+    for name in ("hmc_dense64", "hmc_dense1024"):
+        o = run_reference_hmc_big(name)
+        np.savez_compressed(os.path.join(GOLD, "ref_%s_l50.npz" % name),
+                            **{k: o[k] for k in BIG_KEYS})
+        print("ref_%s_l50 step sizes" % name, o["step_size"].tolist())
+
+
 HMC_CASES = {
     "ref_hmc_diag": ("diag", 12, 16, dict(step_size=1e-3, n_leapfrogs=5,
                                           target_acceptance_rate=0.9, mass_collect_iters=4,
@@ -546,6 +561,26 @@ HMC_CASES = {
                                               target_acceptance_rate=0.8, mass_collect_iters=3,
                                               mass_decay=0.99), 16, 12, 404),
 }
+
+
+def array_digest(a):
+    """SHA-256 of an array's dtype, shape and bytes: equal digests = bit-identical arrays."""
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(("%s %s " % (a.dtype.str, a.shape)).encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def reference_digests():
+    """{fixture: {array: array_digest}} of a fresh run of every tests/golden/ref_*.npz that main()
+    writes (the L = 50 runs aside) -> tests/golden/ref_digests.json, so that the committed
+    fixtures can be checked against what the reference's code produced without its checkout."""
+    runs = {name: (lambda c=c: run_reference_hmc(*c)) for name, c in HMC_CASES.items()}
+    runs.update(ref_vae=run_reference_variational, ref_lntm_hmc=run_reference_lntm_hmc,
+                ref_bnn_sghmc=run_reference_bnn_sghmc, ref_ais=run_reference_ais,
+                ref_sgmcmc=run_reference_sgmcmc)
+    return {name: {k: array_digest(v) for k, v in sorted(run().items())}
+            for name, run in runs.items()}
 
 
 def main():
@@ -570,6 +605,10 @@ def main():
     out = run_reference_sgmcmc()
     np.savez_compressed(os.path.join(GOLD, "ref_sgmcmc.npz"), **out)
     print("ref_sgmcmc draws per step", {k: out[k].tolist() for k in out if k.endswith("_n_used")})
+    write_reference_hmc_big()
+    with open(os.path.join(GOLD, "ref_digests.json"), "w") as f:
+        json.dump(reference_digests(), f, indent=1, sort_keys=True)
+        f.write("\n")
 
 
 if __name__ == "__main__":

@@ -232,7 +232,7 @@ def make_hmc_dense_big(name):
     h = OH.HMC(step_size=cfg["eps0"], n_leapfrogs=L, adapt_step_size=True, adapt_mass=True,
                mass_collect_iters=cfg["mci"])
     keys = ("noise_u", "acc", "accept", "step_size", "eps_used", "mass", "lp", "lp0", "h0",
-            "h1", "acc64", "h0_64", "h1_64", "q_sub", "q_rowsum", "prop_sub64", "n_pushed")
+            "h1", "acc64", "h0_64", "h1_64", "q_sub", "q_rowsum", "n_pushed")
     rec = {k: [] for k in keys}
     stride = D // 16
     for i in range(cfg["iters"]):
@@ -256,7 +256,7 @@ def make_hmc_dense_big(name):
         nu = pushed.astype(np.float32)
         with np.errstate(all="ignore"):
             q_out, info = h.step([q_in.copy()], m32.logp, m32.grad, [npz], nu, adapt, adapt)
-        h0_64, h1_64, acc64, prop64 = _iteration_f64(m64, q_in, npz, info.mass[0].reshape(-1),
+        h0_64, h1_64, acc64, _ = _iteration_f64(m64, q_in, npz, info.mass[0].reshape(-1),
                                                      info.step_size_used, L)
         assert not np.any(np.abs(nu - info.acceptance_rate) < g / 2)
         assert np.array_equal(nu < acc64.astype(np.float32), info.if_accept)
@@ -275,7 +275,6 @@ def make_hmc_dense_big(name):
         rec["h1_64"].append(h1_64)
         rec["q_sub"].append(q_out[0][:, ::stride].copy())
         rec["q_rowsum"].append(q_out[0].astype(np.float64).sum(1))
-        rec["prop_sub64"].append(prop64[:, ::stride].copy())
         rec["n_pushed"].append(np.int32(near.sum()))
     out = {k: np.stack(v) for k, v in rec.items()}
     out["n_search_iters"] = np.int32(h.n_search_iters)

@@ -9,8 +9,9 @@ reference's code, not from the restatement in oracle/.  Here:
 
 * oracle/hmc.py and oracle/sgmcmc.py must reproduce those vectors (float32: bit-exact for the
   element-wise models, rounding of the matmul summation order for the dense one);
-* where the reference checkout is present (this container, not the GPU box) the vectors are
-  regenerated and must equal the committed files bit for bit.
+* the committed files must equal, bit for bit, the reference run whose digests are stored in
+  tests/golden/ref_digests.json (and, where ZHUSUAN_REFERENCE names a checkout of the original
+  ZhuSuan, a fresh run of it).
 
 CPU only.
 """
@@ -27,8 +28,8 @@ from oracle import sgmcmc as OS
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = os.path.join(HERE, "golden")
 SHIM = os.path.join(os.path.dirname(HERE), "oracle", "tf_shim")
-REF = os.environ.get("ZHUSUAN_REFERENCE", "/root/reference")
-have_ref = os.path.isfile(os.path.join(REF, "zhusuan", "hmc.py"))
+REF = os.environ.get("ZHUSUAN_REFERENCE", "")
+have_ref = bool(REF) and os.path.isfile(os.path.join(REF, "zhusuan", "hmc.py"))
 
 
 def _model(g):
@@ -153,43 +154,30 @@ def test_reference_run_equals_oracle_made_fixtures():
         np.testing.assert_allclose(o["q"], r["q"], rtol=tol * 30, atol=tol)
 
 
-@pytest.mark.skipif(not have_ref, reason="reference checkout not present (GPU box)")
 def test_committed_vectors_are_what_the_reference_code_produces():
+    """tests/golden/ref_digests.json: digests of every array of the reference's own run
+    (make_ref_golden.py::reference_digests).  Every committed ref_*.npz must hold exactly those
+    arrays, bit for bit; where ZHUSUAN_REFERENCE names a checkout of the original ZhuSuan, its
+    source is run again and must reproduce the same digests."""
+    import json
+    want = json.load(open(os.path.join(GOLD, "ref_digests.json")))
+    # ref_hmc_diag: the model of examples/toy_examples/gaussian.py built with the reference's own
+    # meta_bayesian_net / BayesianNet.normal / Normal.log_prob; dense32 / dense64: a callable
+    assert sorted(want) == ["ref_ais", "ref_bnn_sghmc", "ref_hmc_dense32", "ref_hmc_dense64",
+                            "ref_hmc_diag", "ref_lntm_hmc", "ref_sgmcmc", "ref_vae"]
     sys.path.insert(0, SHIM)
     saved = {k: sys.modules.get(k) for k in ("tensorflow", "zhusuan")}
     try:
         import make_ref_golden as M
-        # ref_hmc_diag: the model of examples/toy_examples/gaussian.py built with the reference's
-        # own meta_bayesian_net / BayesianNet.normal / Normal.log_prob; dense32: a callable
-        for name in ("ref_hmc_diag", "ref_hmc_dense32"):
-            kind, D, C, cfg, n_iters, n_adapt, seed = M.HMC_CASES[name]
-            out = M.run_reference_hmc(kind, D, C, cfg, n_iters, n_adapt, seed)
+        for name, digests in want.items():
             g = np.load(os.path.join(GOLD, name + ".npz"))
-            for k in ("q", "acc", "step_size", "lp", "h0", "h1", "lp0", "p0", "accept",
-                      "noise_p"):
-                np.testing.assert_array_equal(out[k], g[k], err_msg=name + " " + k)
-        out = M.run_reference_sgmcmc()
-        g = np.load(os.path.join(GOLD, "ref_sgmcmc.npz"))
-        for k in g.files:
-            np.testing.assert_array_equal(out[k], g[k], err_msg=k)
-        out = M.run_reference_ais()
-        g = np.load(os.path.join(GOLD, "ref_ais.npz"))
-        for k in g.files:
-            np.testing.assert_array_equal(out[k], g[k], err_msg=k)
-        out = M.run_reference_variational()
-        g = np.load(os.path.join(GOLD, "ref_vae.npz"))
-        for k in g.files:
-            np.testing.assert_array_equal(out[k], g[k], err_msg=k)
-        out = M.run_reference_bnn_sghmc()
-        g = np.load(os.path.join(GOLD, "ref_bnn_sghmc.npz"))
-        for k in g.files:
-            np.testing.assert_array_equal(out[k], g[k], err_msg=k)
-        out = M.run_reference_lntm_hmc()
-        g = np.load(os.path.join(GOLD, "ref_lntm_hmc.npz"))
-        for k in g.files:
-            np.testing.assert_array_equal(out[k], g[k], err_msg=k)
-        import zhusuan.hmc
-        assert os.path.realpath(zhusuan.hmc.__file__).startswith(os.path.realpath(REF))
+            assert sorted(g.files) == sorted(digests), name
+            for k in g.files:
+                assert M.array_digest(g[k]) == digests[k], name + " " + k
+        if have_ref:
+            assert M.reference_digests() == want
+            import zhusuan.hmc
+            assert os.path.realpath(zhusuan.hmc.__file__).startswith(os.path.realpath(REF))
     finally:
         sys.path.remove(SHIM)
         for k in [m for m in sys.modules if m == "tensorflow" or m.startswith("zhusuan")]:
@@ -344,28 +332,16 @@ def test_oracle_lntm_hmc_follows_reference_run():
         q = [g["eta"][i].copy()]             # continue from the reference's state
 
 
-@pytest.mark.skipif(not have_ref, reason="reference checkout not present (GPU box)")
 @pytest.mark.parametrize("name", ["hmc_dense64", "hmc_dense1024"])
 def test_reference_hmc_itself_passes_the_l50_protocol(name):
     """The L = 50 adaptive fixtures the benchmarked CUDA kernels are replayed against
     (tests/golden/hmc_dense64.npz, hmc_dense1024.npz: written by the float32 oracle, with a
     float64 re-evaluation of every iteration) versus THE REFERENCE'S OWN hmc.py run on the TF
-    stand-in under the same protocol, at the benchmark's shape (D = 1024, L = 50, both step-size
-    searches, mass != 1): every accept decision, the step-size trajectory exactly, Hamiltonians
-    within 1e-6 of float64."""
-    sys.path.insert(0, SHIM)
-    saved = {k: sys.modules.get(k) for k in ("tensorflow", "zhusuan")}
-    try:
-        import make_ref_golden as M
-        o = M.run_reference_hmc_big(name)
-    finally:
-        sys.path.remove(SHIM)
-        for k in [m for m in sys.modules if m == "tensorflow" or m.startswith("tensorflow.")
-                  or m.startswith("zhusuan")]:
-            del sys.modules[k]
-        for k, v in saved.items():
-            if v is not None:
-                sys.modules[k] = v
+    stand-in under the same protocol (tests/golden/ref_<name>_l50.npz, written by
+    make_ref_golden.py::write_reference_hmc_big), at the benchmark's shape (D = 1024, L = 50,
+    both step-size searches, mass != 1): every accept decision, the step-size trajectory
+    exactly, Hamiltonians within 1e-6 of float64."""
+    o = np.load(os.path.join(GOLD, "ref_%s_l50.npz" % name))
     g = np.load(os.path.join(GOLD, name + ".npz"))
     accept = (g["noise_u"] < o["acc"]).astype(np.int32)
     np.testing.assert_array_equal(accept, g["accept"])
